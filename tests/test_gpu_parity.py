@@ -1,6 +1,7 @@
 """GPU parity tests (-m gpu): every CUDA entry point, called through the C ABI via the host API,
-against (a) the CPU oracle, (b) the committed golden vectors and (c) -- when oracle/_ref was
-shipped -- the reference's own CUDA kernels compiled for sm_100a.
+against (a) the CPU oracle, (b) the committed golden vectors and (c) the outputs of the reference's
+own CUDA kernels (compiled for sm_100a) on the same inputs, stored in tests/golden/reference_kernels.npz
+by tests/golden/make_reference_kernels.py.
 Tolerances: bit-exact for NMS indices / panoptic label maps / FPN levels; fp32 outputs within 1e-3
 (BASELINE.json north_star), in practice ~1e-5 for the fp32 tiles."""
 import os
@@ -23,10 +24,17 @@ def dev():
 
 @pytest.fixture(scope="module")
 def ref():
-    try:
-        return O.RefKernels()
-    except (FileNotFoundError, OSError):
-        return None
+    return np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_kernels.npz"))
+
+
+REF_SAMPLE = 2048
+
+
+def ref_sample(n):
+    """Fixed subset of a flattened output of n elements: large reference-kernel outputs are stored at these indices."""
+    if n <= REF_SAMPLE:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(n).choice(n, REF_SAMPLE, replace=False))
 
 
 def t(a, dev):
@@ -56,27 +64,27 @@ def test_roi_align_golden(dev, golden_ops, ref):
     g = golden_ops
     out = U.roi_align(t(g["ra_feat"], dev), t(g["ra_rois"], dev), 7, 7, 0.25).cpu().numpy()
     assert np.abs(out - g["ra_out"]).max() < 1e-4
-    if ref is not None:
-        r = ref.roi_align(t(g["ra_feat"], dev), t(g["ra_rois"], dev), 7, 7, 0.25).cpu().numpy()
-        assert np.abs(out - r).max() < 1e-4
+    assert np.abs(out - ref["roi_align_golden"]).max() < 1e-4
+
+
+def roi_align_config1_case():
+    torch.manual_seed(0)
+    rng = np.random.default_rng(0)
+    return torch.randn(1, 256, 256, 256), rand_rois(rng, 32, 1, 1024, 16, 512)
 
 
 @pytest.mark.parametrize("ph", [7, 14])
 def test_roi_align_config1_nchw_and_nhwc(dev, ph, ref):
     """BASELINE config #1: 1x256x256x256 feature map, 32 boxes, scale 1/4, sampling_ratio 2."""
     import upsnet_b200 as U
-    torch.manual_seed(0)
-    rng = np.random.default_rng(0)
-    feat = torch.randn(1, 256, 256, 256)
-    rois = rand_rois(rng, 32, 1, 1024, 16, 512)
+    feat, rois = roi_align_config1_case()
     want = O.roi_align(feat.numpy(), rois, ph, ph, 0.25)
     f = feat.to(dev); r = t(rois, dev)
     got = U.RoIAlign(ph, ph, 0.25)(f, r).cpu().numpy()
     assert np.abs(got - want).max() < 1e-4  # FMA contraction moves sample coords by 1 ulp
     got_nhwc = U.roi_align(f.permute(0, 2, 3, 1).contiguous(), r, ph, ph, 0.25, layout="nhwc")
     assert np.abs(got_nhwc.permute(0, 3, 1, 2).cpu().numpy() - want).max() < 1e-4
-    if ref is not None:
-        assert np.abs(ref.roi_align(f, r, ph, ph, 0.25).cpu().numpy() - got).max() < 1e-4
+    assert np.abs(ref["roi_align_config1_ph%d" % ph] - got.reshape(-1)[ref_sample(got.size)]).max() < 1e-4
 
 
 def test_roi_align_edge_cases(dev):
@@ -126,24 +134,27 @@ def test_nms_golden_reference_py_cpu_nms(dev, golden_ref, ref):
         d = g["nms%d_dets" % i]; thr = float(g["nms%d_thresh" % i])
         keep = U.gpu_nms_wrapper(thr, 0)(d)
         assert keep == g["nms%d_keep" % i].tolist(), "case %d" % i
-        if ref is not None:
-            assert ref.nms(d, thr) == keep
+        assert ref["nms_golden_%d" % i].tolist() == keep
 
 
-def test_nms_dense_random_bit_exact(dev, ref):
-    import upsnet_b200 as U
+def nms_dense_cases():
     rng = np.random.default_rng(11)
     for n, extent in [(1, 50), (64, 80), (65, 80), (129, 100), (1000, 250), (4097, 600), (8000, 1200)]:
         c = rng.uniform(0, extent, (n, 2)); s = np.exp(rng.uniform(np.log(16), np.log(128), (n, 2)))
         scores = (rng.permutation(n) + 1.0) / (n + 1)
-        d = np.concatenate([c - s / 2, c + s / 2, scores[:, None]], 1).astype(np.float32)
+        yield n, np.concatenate([c - s / 2, c + s / 2, scores[:, None]], 1).astype(np.float32)
+
+
+def test_nms_dense_random_bit_exact(dev, ref):
+    import upsnet_b200 as U
+    for n, d in nms_dense_cases():
         for thr in (0.3, 0.5, 0.7):
             want = O.nms(d, thr)
             got = U.nms(t(d[:, :4], dev), t(d[:, 4], dev), thr).cpu().tolist()
             assert got == want, (n, thr)
             assert len(want) < n or n == 1
-        if ref is not None and n <= 4097:
-            assert ref.nms(d, 0.5) == O.nms(d, 0.5)
+        if n <= 4097:
+            assert ref["nms_dense_%d" % n].tolist() == O.nms(d, 0.5)
 
 
 def test_nms_segmented_levels_one_launch(dev):
@@ -190,20 +201,19 @@ def test_dcn_golden(dev, golden_ops, ref):
     m.weight.data.copy_(w); m.bias.data.copy_(b)
     y2 = m(x, t(g["dcn2_om"], dev)).detach().cpu().numpy()      # module call = autograd path (parameters require grad), like the reference
     assert np.abs(y2 - g["dcn2_y"]).max() < 1e-4
-    if ref is not None:
-        r = ref.deform_conv(x, t(g["dcn_off"], dev), w, b, pad=1, dg=2).cpu().numpy()
-        assert np.abs(y - r).max() < 1e-4
+    assert np.abs(y - ref["dcn_golden"]).max() < 1e-4
 
 
-@pytest.mark.parametrize("cfg", [
+DCN_CFGS = [
     dict(N=1, Cin=256, Cout=128, H=32, W=48, stride=1, pad=1, dil=1, dg=1),   # semantic-head layer shape (a12)
     dict(N=2, Cin=64, Cout=96, H=25, W=42, stride=1, pad=1, dil=1, dg=1),     # ragged spatial size (B: 25x42)
     dict(N=2, Cin=32, Cout=40, H=17, W=19, stride=2, pad=1, dil=1, dg=2),
     dict(N=1, Cin=16, Cout=16, H=20, W=20, stride=1, pad=2, dil=2, dg=4),
-])
-@pytest.mark.parametrize("modulated", [False, True])
-def test_dcn_vs_oracle(dev, cfg, modulated, ref):
-    import upsnet_b200 as U
+]
+
+
+def dcn_case(cfg, modulated):
+    """(x, offset, weight, bias, mask or None) of one test_dcn_vs_oracle case."""
     rng = np.random.default_rng(21)
     N, Cin, Cout, H, W = cfg["N"], cfg["Cin"], cfg["Cout"], cfg["H"], cfg["W"]
     Ho = O.conv_out(H, cfg["pad"], cfg["dil"], 3, cfg["stride"]); Wo = O.conv_out(W, cfg["pad"], cfg["dil"], 3, cfg["stride"])
@@ -212,15 +222,21 @@ def test_dcn_vs_oracle(dev, cfg, modulated, ref):
     b = rng.standard_normal(Cout).astype(np.float32)
     off = (rng.standard_normal((N, 18 * cfg["dg"], Ho, Wo)) * 2.5).astype(np.float32)
     mask = (rng.uniform(0, 2, (N, 9 * cfg["dg"], Ho, Wo))).astype(np.float32) if modulated else None
+    return x, off, w, b, mask
+
+
+@pytest.mark.parametrize("cfg", DCN_CFGS)
+@pytest.mark.parametrize("modulated", [False, True])
+def test_dcn_vs_oracle(dev, cfg, modulated, ref):
+    import upsnet_b200 as U
+    x, off, w, b, mask = dcn_case(cfg, modulated)
     want = O.deform_conv(x, off, w, b, mask, cfg["stride"], cfg["pad"], cfg["dil"], cfg["dg"])
     got = U.deform_conv(t(x, dev), t(off, dev), t(w, dev), t(b, dev), cfg["stride"], cfg["pad"], cfg["dil"],
                         cfg["dg"], mask=None if mask is None else t(mask, dev)).cpu().numpy()
     assert np.abs(got - want).max() < TOL, np.abs(got - want).max()
     assert np.abs(got - want).max() < 1e-4  # fp32 tiles are far inside the 1e-3 contract
-    if ref is not None:
-        r = ref.deform_conv(t(x, dev), t(off, dev), t(w, dev), t(b, dev),
-                            None if mask is None else t(mask, dev), cfg["stride"], cfg["pad"], cfg["dil"], cfg["dg"])
-        assert np.abs(got - r.cpu().numpy()).max() < TOL
+    r = ref["dcn_cfg%d_mod%d" % (DCN_CFGS.index(cfg), modulated)]
+    assert np.abs(got.reshape(-1)[ref_sample(got.size)] - r).max() < TOL
 
 
 def test_deform_conv_with_offset_module_and_state_dict_names(dev):
